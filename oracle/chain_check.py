@@ -19,11 +19,75 @@ import numpy as np
 from qnnpack_b200 import mobilenet_v2 as M
 
 
+class _OracleOp:
+    def __init__(self, kind, args):
+        self.kind, self.args, self.io = kind, args, None
+
+
+class OracleHost:
+    """The operators of the MobileNetV2 graph (convolution, fully connected, add, global average pooling) on the C oracle
+    and the NumPy restatement of the eltwise operators, behind the part of the qnnpack.h driver that the gate uses.
+    Both restatements are pinned to the unmodified reference by the CPU tests (tests/test_oracle.py,
+    tests/test_ops_oracle.py), so this is the reference chain wherever oracle/_ref has not been built."""
+
+    def __init__(self):
+        from oracle import q8_oracle as O
+        self.c = O.COracle()
+
+    def create_convolution(self, kernel, bias, **kw):
+        return 0, _OracleOp("conv", (np.array(kernel, np.uint8), np.array(bias, np.int32), kw))
+
+    def create_fully_connected(self, kernel, bias, **kw):
+        return 0, _OracleOp("fc", (np.array(kernel, np.uint8), np.array(bias, np.int32), kw))
+
+    def create(self, name, *args):
+        return 0, _OracleOp(name, args)
+
+    def setup_convolution(self, op, batch, in_h, in_w, x, in_stride, out, out_stride):
+        op.io = (batch, in_h, in_w, x, in_stride, out, out_stride)
+        return 0
+
+    def setup_fully_connected(self, op, batch, x, in_stride, out, out_stride):
+        op.io = (batch, x, in_stride, out, out_stride)
+        return 0
+
+    def setup(self, name, op, *args):
+        op.io = args
+        return 0
+
+    def run(self, op):
+        from oracle import q8_ops_oracle as OPS
+        if op.kind == "conv":
+            (n, h, w, x, xs, out, ys), (k, b, kw) = op.io, op.args
+            y = self.c.convolution(x[:n * h * w * xs].reshape(n, h, w, xs), k, b, out_stride=ys, **kw)
+        elif op.kind == "fc":
+            (n, x, xs, out, ys), (k, b, kw) = op.io, op.args
+            y = self.c.fully_connected(x[:n * xs].reshape(n, xs), k, b, out_stride=ys, **kw)
+        elif op.kind == "add_nc_q8":
+            (n, a, a_s, b, b_s, out, ys), (c, *q) = op.io, op.args
+            assert a_s == b_s == ys == c
+            y = OPS.add(a[:n * c], b[:n * c], OPS.add_params(*q))
+        elif op.kind == "global_average_pooling_nwc_q8":
+            (n, width, x, xs, out, ys), (c, izp, iscale, ozp, oscale, qmin, qmax) = op.io, op.args
+            assert xs == ys == c
+            y = OPS.global_average_pooling(x[:n * width * c].reshape(n, width, c), izp, iscale, ozp, oscale, qmin, qmax)
+        else:
+            raise NotImplementedError(op.kind)
+        out[:y.size] = y.reshape(-1)
+        return 0
+
+    def delete(self, op):
+        return 0
+
+    def close(self):
+        pass
+
+
 def _host_lib():
     from oracle import ref as R
     if R.available():
         return R.QnnpackHost(), "oracle/_ref (unmodified reference, SSE2 ukernels)"
-    raise RuntimeError("oracle/_ref/libqnnpack_ref.so is missing (make -C oracle ref)")
+    return OracleHost(), "oracle/q8_oracle.c + q8_ops_oracle.py (restatements pinned to the reference)"
 
 
 def _srcs(nodes, i):

@@ -1,11 +1,13 @@
-"""GPU parity of the operators beside the convolution path (SURVEY.md §8f rows 1, 3, 4) against the UNMODIFIED reference
-compiled into oracle/_ref: add, global average pooling, average / max pooling, clamp, sigmoid, leaky ReLU, softargmax,
+"""GPU parity of the operators beside the convolution path (SURVEY.md §8f rows 1, 3, 4) against what the UNMODIFIED
+reference computed for the same calls (tests/reference.py): add, global average pooling, average / max pooling, clamp, sigmoid, leaky ReLU, softargmax,
 channel shuffle, deconvolution.  Case grids restate test/add.cc, test/global-average-pooling.cc, test/average-pooling.cc,
 test/max-pooling.cc, test/clamp.cc, test/sigmoid.cc, test/leaky-relu.cc, test/softargmax.cc, test/channel-shuffle.cc and
 test/deconvolution.cc with fixed seeds (the reference draws from std::random_device).  Byte-exact, gaps between rows
 (0xA5 canary) untouched."""
 import numpy as np
 import pytest
+
+from tests import reference as REF
 
 pytestmark = pytest.mark.gpu
 
@@ -42,20 +44,21 @@ NC_SHAPES = [(1, 1, 0, 0), (1, 100, 0, 0), (3, 5, 0, 0), (3, 100, 0, 0), (3, 100
 @pytest.mark.parametrize("batch,channels,xe,ye", NC_SHAPES)
 @pytest.mark.parametrize("q", [dict(), dict(a_zp=0, b_zp=255, y_zp=3), dict(a_scale=0.25, b_scale=4.0, y_scale=1.3),
                                dict(qmin=128), dict(qmax=128), dict(a_scale=0.004, b_scale=2.3, y_scale=0.9)])
-def test_add(gpu_lib, ref_lib, batch, channels, xe, ye, q):
+def test_add(gpu_lib, batch, channels, xe, ye, q):
     rng = np.random.default_rng(batch * 1000 + channels)
     a = _rows(rng, batch, channels, channels + xe)
     b = _rows(rng, batch, channels, channels + xe + 1)
     args = (channels, q.get("a_zp", 121), np.float32(q.get("a_scale", 0.75)), q.get("b_zp", 127), np.float32(q.get("b_scale", 1.25)),
             q.get("y_zp", 133), np.float32(q.get("y_scale", 1.96875)), q.get("qmin", 0), q.get("qmax", 255))
-    out = [_run_nc(l, "add_nc_q8", args, batch, channels, a, channels + xe, channels + ye, b, channels + xe + 1)
-           for l in (gpu_lib, ref_lib)]
-    assert np.array_equal(out[0], out[1])
-    assert (out[0][:, channels:] == 0xA5).all()
+    def run(l):
+        return _run_nc(l, "add_nc_q8", args, batch, channels, a, channels + xe, channels + ye, b, channels + xe + 1)
+    got = run(gpu_lib)
+    REF.expect(got, run)
+    assert (got[:, channels:] == 0xA5).all()
 
 
 @pytest.mark.parametrize("batch,channels,xe,ye", NC_SHAPES)
-def test_clamp_lut_ops(gpu_lib, ref_lib, batch, channels, xe, ye):
+def test_clamp_lut_ops(gpu_lib, batch, channels, xe, ye):
     rng = np.random.default_rng(batch * 77 + channels)
     x = _rows(rng, batch, channels, channels + xe)
     cases = [("clamp_nc_u8", (channels, 0, 255)), ("clamp_nc_u8", (channels, 128, 255)), ("clamp_nc_u8", (channels, 17, 200)),
@@ -66,21 +69,23 @@ def test_clamp_lut_ops(gpu_lib, ref_lib, batch, channels, xe, ye):
              ("softargmax_nc_q8", (channels, np.float32(0.176080), 0, np.float32(1.0 / 256.0))),
              ("softargmax_nc_q8", (channels, np.float32(0.01), 0, np.float32(1.0 / 256.0)))]
     for name, args in cases:
-        out = [_run_nc(l, name, args, batch, channels, x, channels + xe, channels + ye) for l in (gpu_lib, ref_lib)]
-        assert np.array_equal(out[0], out[1]), (name, args)
-        assert (out[0][:, channels:] == 0xA5).all()
+        got = _run_nc(gpu_lib, name, args, batch, channels, x, channels + xe, channels + ye)
+        REF.expect(got, lambda l: _run_nc(l, name, args, batch, channels, x, channels + xe, channels + ye), f"{name}{args}")
+        assert (got[:, channels:] == 0xA5).all()
 
 
 @pytest.mark.parametrize("groups,gc", [(2, 1), (2, 37), (3, 5), (4, 16), (5, 7), (7, 24), (2, 160)])
 @pytest.mark.parametrize("batch,xe,ye", [(1, 0, 0), (3, 0, 0), (3, 5, 0), (3, 0, 9)])
-def test_channel_shuffle(gpu_lib, ref_lib, groups, gc, batch, xe, ye):
+def test_channel_shuffle(gpu_lib, groups, gc, batch, xe, ye):
     channels = groups * gc
     rng = np.random.default_rng(groups * 100 + gc)
     x = _rows(rng, batch, channels, channels + xe)
-    out = [_run_nc(l, "channel_shuffle_nc_x8", (groups, gc), batch, channels, x, channels + xe, channels + ye) for l in (gpu_lib, ref_lib)]
-    assert np.array_equal(out[0], out[1])
+    def run(l):
+        return _run_nc(l, "channel_shuffle_nc_x8", (groups, gc), batch, channels, x, channels + xe, channels + ye)
+    got = run(gpu_lib)
+    REF.expect(got, run)
     want = x[:, :channels].reshape(batch, groups, gc).transpose(0, 2, 1).reshape(batch, channels)
-    assert np.array_equal(out[0][:, :channels], want)
+    assert np.array_equal(got[:, :channels], want)
 
 
 def _run_gavg(lib, batch, width, channels, x, x_stride, y_stride, q):
@@ -98,7 +103,7 @@ def _run_gavg(lib, batch, width, channels, x, x_stride, y_stride, q):
                                                         (3, 5, 13, 4, 0), (3, 8, 24, 0, 5), (2, 14, 9, 0, 0), (5, 100, 36, 0, 0),
                                                         (2, 7, 1, 0, 0), (4, 23, 128, 8, 8)])
 @pytest.mark.parametrize("q", [dict(), dict(izp=0, ozp=255), dict(**{"is": 0.01}, os=1.7), dict(qmin=128), dict(qmax=128)])
-def test_global_average_pooling(gpu_lib, ref_lib, batch, width, channels, xe, ye, q):
+def test_global_average_pooling(gpu_lib, batch, width, channels, xe, ye, q):
     qq = dict(izp=121, ozp=133, qmin=0, qmax=255, **{"is": 1.0}, os=1.0)
     qq.update(q)
     rng = np.random.default_rng(width * 31 + channels)
@@ -106,8 +111,9 @@ def test_global_average_pooling(gpu_lib, ref_lib, batch, width, channels, xe, ye
     x = np.zeros(16 + batch * width * xs + 16, np.uint8)
     xv = x[16:16 + batch * width * xs]
     xv[...] = rng.integers(0, 256, xv.size, dtype=np.uint8)
-    out = [_run_gavg(l, batch, width, channels, xv, xs, channels + ye, qq) for l in (gpu_lib, ref_lib)]
-    assert np.array_equal(out[0], out[1])
+    def run(l):
+        return _run_gavg(l, batch, width, channels, xv, xs, channels + ye, qq)
+    REF.expect(run(gpu_lib), run)
 
 
 def _run_pool(lib, kind, n, h, w, c, xs, ys, x, pad, pool, stride, dil, q):
@@ -144,7 +150,7 @@ POOL_CASES = [
 
 @pytest.mark.parametrize("case", POOL_CASES, ids=lambda c: "x".join(str(v) for v in c[:4]) + f"_p{c[7][0]}x{c[7][1]}")
 @pytest.mark.parametrize("kind", ["avg", "max"])
-def test_pooling(gpu_lib, ref_lib, case, kind):
+def test_pooling(gpu_lib, case, kind):
     n, h, w, c, xe, ye, pad, pool, stride, dil = case
     rng = np.random.default_rng(h * 100 + w + c)
     xs, ys = c + xe, c + ye
@@ -154,14 +160,14 @@ def test_pooling(gpu_lib, ref_lib, case, kind):
     for q in (dict(), dict(izp=3, ozp=200, **{"is": 0.3}, os=0.11), dict(qmin=100, qmax=180)):
         qq = dict(izp=121, ozp=133, qmin=0, qmax=255, **{"is": 1.0}, os=1.0)
         qq.update(q)
-        out = [_run_pool(l, kind, n, h, w, c, xs, ys, x, pad, pool, stride, dil, qq) for l in (gpu_lib, ref_lib)]
-        assert np.array_equal(out[0], out[1]), (kind, q)
+        got = _run_pool(gpu_lib, kind, n, h, w, c, xs, ys, x, pad, pool, stride, dil, qq)
+        REF.expect(got, lambda l: _run_pool(l, kind, n, h, w, c, xs, ys, x, pad, pool, stride, dil, qq), f"{kind} {q}")
     if kind == "max":  # dilated windows: padded taps read the clamped edge pixel (src/indirection.c:218-224)
         for d in ((2, 2), (1, 3)):
             if (pool[0] - 1) * d[0] + 1 <= h + pad[0] + pad[2] and (pool[1] - 1) * d[1] + 1 <= w + pad[1] + pad[3]:
                 qq = dict(qmin=0, qmax=255)
-                out = [_run_pool(l, kind, n, h, w, c, xs, ys, x, pad, pool, stride, d, qq) for l in (gpu_lib, ref_lib)]
-                assert np.array_equal(out[0], out[1]), ("max dilated", d)
+                got = _run_pool(gpu_lib, kind, n, h, w, c, xs, ys, x, pad, pool, stride, d, qq)
+                REF.expect(got, lambda l: _run_pool(l, kind, n, h, w, c, xs, ys, x, pad, pool, stride, d, qq), f"max dilated {d}")
 
 
 def _run_deconv(lib, x, k, b, n, h, w, groups, gic, goc, pad, adj, ks, stride, dil, q, ye):
@@ -191,7 +197,7 @@ DECONV_CASES = [
 
 
 @pytest.mark.parametrize("case", DECONV_CASES, ids=lambda c: f"{c[1]}x{c[2]}_g{c[3]}_k{c[8][0]}x{c[8][1]}_s{c[9][0]}x{c[9][1]}_d{c[10][0]}")
-def test_deconvolution(gpu_lib, ref_lib, case):
+def test_deconvolution(gpu_lib, case):
     n, h, w, groups, gic, goc, pad, adj, ks, stride, dil, ye = case
     rng = np.random.default_rng(h * 10 + w + gic)
     buf = np.zeros(16 + n * h * w * groups * gic + 16, np.uint8)
@@ -202,5 +208,5 @@ def test_deconvolution(gpu_lib, ref_lib, case):
     for q in (dict(), dict(izp=0, kzp=255), dict(qmin=128), dict(qmax=128)):
         qq = dict(izp=127, kzp=127, ozp=127, qmin=0, qmax=255, os=float(ks[0] * ks[1] * gic * 40.0))
         qq.update(q)
-        out = [_run_deconv(l, x, k, b, n, h, w, groups, gic, goc, pad, adj, ks, stride, dil, qq, ye) for l in (gpu_lib, ref_lib)]
-        assert np.array_equal(out[0], out[1]), q
+        got = _run_deconv(gpu_lib, x, k, b, n, h, w, groups, gic, goc, pad, adj, ks, stride, dil, qq, ye)
+        REF.expect(got, lambda l: _run_deconv(l, x, k, b, n, h, w, groups, gic, goc, pad, adj, ks, stride, dil, qq, ye), str(q))

@@ -1,13 +1,14 @@
 """CPU tests: the oracle (C restatement + NumPy restatement) against
   (a) the reference's deterministic Q31 known-answer tests (test/requantization-tester.h),
   (b) golden vectors generated from the unmodified compiled reference (tests/golden/),
-  (c) the compiled reference itself when oracle/_ref is present.
+  (c) what the compiled reference computed for the same calls (tests/reference.py), and the compiled reference itself
+      where oracle/_ref has been built.
 """
 import numpy as np
 import pytest
 
 from oracle import q8_oracle as O
-from tests import cases as CS, util as U
+from tests import cases as CS, reference as REF, util as U
 
 
 # ---- (a) Q31 known-answer tests, restated from test/requantization-tester.h ---------------------
@@ -115,7 +116,7 @@ def test_numpy_oracle_matches_golden_mobilenet(golden, entry):
     assert U.digest(y) == str(golden[f"mnv2/{case['name']}/y_digest"])
 
 
-# ---- (c) the compiled reference itself, where it exists -------------------------------------------
+# ---- (c) the compiled reference: recorded, and itself where it exists ------------------------------
 @pytest.mark.parametrize("case", CS.OPERATOR_CASES[::4] + CS.DW_UKERNEL_CASES[::4], ids=lambda c: c["name"])
 def test_compiled_reference_matches_golden(ref_lib, golden, case):
     x, k, b, kw = U.conv_setup(case)
@@ -123,17 +124,17 @@ def test_compiled_reference_matches_golden(ref_lib, golden, case):
 
 
 @pytest.mark.parametrize("case", CS.DW_TC_CASES + CS.STEM_CASES + CS.PERSISTENT_CASES, ids=lambda c: c["name"])
-def test_oracle_matches_compiled_reference_on_device_path_cases(ref_lib, oracle_c, case):
+def test_oracle_matches_compiled_reference_on_device_path_cases(oracle_c, case):
     """The GPU tests compare these shapes (tcgen05 depthwise classes, stem loaders, long item sequences) with the C oracle;
     here the oracle is pinned to the unmodified reference on exactly the same inputs."""
     x, k, b, kw = U.conv_setup(case)
-    U.assert_same_bytes(U.run_conv(oracle_c, case, x, k, b, kw), U.run_conv(ref_lib, case, x, k, b, kw), case["name"])
+    REF.expect(U.run_conv(oracle_c, case, x, k, b, kw), lambda l: U.run_conv(l, case, x, k, b, kw), case["name"])
 
 
-def test_compiled_reference_q31_matches_oracle(ref_lib, oracle_c):
+def test_compiled_reference_q31_matches_oracle(oracle_c):
     rng = np.random.default_rng(3)
     x = rng.integers(-(2**31), 2**31, 1 << 16, dtype=np.int64).astype(np.int32)
     for scale, zp, qmin, qmax in ((0.75, 127, 1, 254), (2.0 ** -11 * 1.3, 3, 0, 255), (2.0 ** -31, 255, 0, 200)):
-        want = ref_lib.requantize_q31(x, scale, zp, qmin, qmax, variant="scalar")
-        assert np.array_equal(ref_lib.requantize_q31(x, scale, zp, qmin, qmax, variant="sse2"), want)
-        assert np.array_equal(oracle_c.requantize_q31(x, scale, zp, qmin, qmax), want)
+        got = oracle_c.requantize_q31(x, scale, zp, qmin, qmax)
+        for variant in ("scalar", "sse2"):
+            REF.expect(got, lambda l: l.requantize_q31(x, scale, zp, qmin, qmax, variant=variant), variant)
