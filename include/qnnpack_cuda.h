@@ -85,6 +85,11 @@ int qnnp_cuda_debug_pack_dwconv(size_t channels, uint8_t input_zero_point, uint8
 int qnnp_cuda_debug_plan_dwconv32(int channels, int batch, int in_h, int in_w, int out_h, int out_w, int stride, int pad_top,
                                   int pad_left, int wmode, int out[48]);
 int qnnp_cuda_debug_pack_dwconv32(size_t channels, uint8_t kernel_zero_point, const uint8_t* kernel, uint8_t* wpack);
+/* Border-class bias table of either form's plan (pair = 0 / 1): out = {bias_smem, bias_off, bias_rstride, bias_nrc, bias_ncc,
+ * bias_rslot, bias_cslot, bias_rcls, bias_ccls, smem_total, num_stages, stage_bytes} (see DwTcParams in
+ * qnnpack_b200/csrc/q8_dwconv_sm100.cuh).  Returns 0 when the shape is not eligible. */
+int qnnp_cuda_debug_plan_dwconv_bias(int channels, int batch, int in_h, int in_w, int out_h, int out_w, int stride, int pad_top,
+                                     int pad_left, int wmode, int pair, int out[12]);
 /* Launches of the depthwise tensor-core kernel since qnnp_initialize() (tests use it to prove the routing). */
 unsigned long long qnnp_cuda_debug_dw_umma_launch_count(void);
 

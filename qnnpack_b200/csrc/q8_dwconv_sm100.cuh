@@ -79,6 +79,14 @@ struct DwTcParams {
   int store32;              // 1: the epilogue pairs channel groups and writes 32 bytes per pixel with one 256-bit store
                             // (needs 32-byte aligned output pixels and an even number of channel groups per item)
   int acc_sign;             // +1, or -1 when the B operand holds kzp - w (the accumulators are the negated sums)
+  // Border-class biases.  The epilogue reads row ((row slot * bias_rstride) + column slot) of a [slots][channels] table; a
+  // class's row / column slot is nibble (row / column class bits) of bias_rslot / bias_cslot.  Global table (bias_smem = 0):
+  // slot = class bits, bias_rstride = 8, i.e. bias_cls itself.  bias_smem = 1: only the bias_nrc x bias_ncc classes the
+  // geometry produces, copied from bias_cls into shared memory at bias_off (from the aligned base) when the CTA starts; slot k's
+  // class bits are nibble k of bias_rcls / bias_ccls, and classes the geometry never produces (rows and columns whose outputs
+  // are not stored) read slot 0.
+  int bias_smem, bias_off, bias_rstride, bias_nrc, bias_ncc;
+  uint32_t bias_rslot, bias_cslot, bias_rcls, bias_ccls;
   // item schedule: a CTA's next item is the NEXT item; in (cb, xtile, ytile, nblk) digits that is this step
   int chunk;                // items per CTA: CTA b runs items [b * chunk, min(total, (b + 1) * chunk))
   int step_cb, step_x, step_y, step_n;

@@ -24,7 +24,9 @@
 //   epilogue: TMEM -> registers, + bias_cls, Q31 requantisation, 16-byte global store per pixel.
 //   bias_cls: the reference pads with the input zero point, TMA pads with 0.  Both agree once the bias carries
 //             -izp * (sum of w - kzp over the taps that are INSIDE the image): 64 border classes (3 row bits x 3
-//             column bits) x channels, built on the host; interior pixels all use class 63.
+//             column bits) x channels, built on the host; interior pixels all use class 63.  The (at most 9, for padding
+//             <= 1 on images >= 3 pixels) classes a geometry produces are copied into shared memory when they fit beside
+//             the ring (DwTcParams::bias_smem): one LDS instead of one LDG per bias word.
 //
 // Same integers as the reference:  acc[c] = bias[c] + sum_valid_taps (a_tap[c] - izp) * (w_tap[c] - kzp).
 #include <cuda.h>
@@ -171,11 +173,20 @@ __device__ __forceinline__ void tma_load_5d(uint32_t dst, const CUtensorMap* tm,
       : "memory");
 }
 
+__device__ __forceinline__ int4 lds128(uint32_t addr) {
+  int4 r;
+  asm volatile("ld.shared.v4.s32 {%0, %1, %2, %3}, [%4];" : "=r"(r.x), "=r"(r.y), "=r"(r.z), "=r"(r.w) : "r"(addr));
+  return r;
+}
+
+__device__ __forceinline__ uint32_t nibble(uint32_t packed, uint32_t k) { return (packed >> (4u * k)) & 15u; }
+
 // One unit = 16 channels of one 8-column sub-tile for the warp's 32 TMEM lanes (4 row groups x 8 columns).
-// The bias words are fetched BEFORE the TMEM load is waited for (the wait is a compiler barrier for memory operations).
-template <int RQ, int NB>
-__device__ __forceinline__ uint4 epilogue_unit(const DwTcParams& p, uint32_t taddr, const int32_t* bias, bool last,
-                                               uint32_t tmem_empty_bar) {
+// The bias words (element `bias_idx` of the border-class table: in shared memory when SMB = p.bias_smem, else bias_cls) are
+// fetched BEFORE the TMEM load is waited for (the wait is a compiler barrier for memory operations).
+template <int RQ, int NB, bool SMB>
+__device__ __forceinline__ uint4 epilogue_unit(const DwTcParams& p, uint32_t taddr, uint32_t bias_idx, uint32_t bias_smem_base,
+                                               bool last, uint32_t tmem_empty_bar) {
   // order: start the (asynchronous) TMEM load, fetch the bias words while it is in flight, then wait — the wait is a
   // compiler barrier for memory operations, so the bias loads must be issued before it
   int32_t v[16];
@@ -187,7 +198,9 @@ __device__ __forceinline__ uint4 epilogue_unit(const DwTcParams& p, uint32_t tad
   }
   int4 b[4];
 #pragma unroll
-  for (int t = 0; t < 4; t++) b[t] = __ldg(reinterpret_cast<const int4*>(bias) + t);
+  for (int t = 0; t < 4; t++)
+    b[t] = SMB ? lds128(bias_smem_base + bias_idx * 4u + 16u * (uint32_t) t)
+                       : __ldg(reinterpret_cast<const int4*>(p.bias_cls + bias_idx) + t);
   tmem_ld_wait();
   if constexpr (NB == 32) {
 #pragma unroll
@@ -378,7 +391,8 @@ __device__ __forceinline__ void mma_role(const DwTcParams& p, Ctl& ctl, const It
   }
 }
 
-template <int S, int RQ, int NB, bool PAIR>
+// SMB = DwTcParams::bias_smem (a template parameter, so that the global-table instances are the plain code)
+template <int S, int RQ, int NB, bool PAIR, bool SMB>
 __global__ void __launch_bounds__(kThreads, 1)
     q8_dwconv3x3_umma_kernel(const __grid_constant__ DwTcParams p, const __grid_constant__ CUtensorMap tmap) {
   extern __shared__ __align__(1024) uint8_t smem_raw[];
@@ -400,6 +414,16 @@ __global__ void __launch_bounds__(kThreads, 1)
     fence_mbar_init();
   }
   if (warp == kMmaWarp) tmem_alloc<kTmemCols>(smem_u32(&ctl.tmem_base));
+  if constexpr (SMB) {  // the border classes this geometry produces, all channels (see DwTcParams::bias_smem)
+    const uint32_t q4 = (uint32_t) p.channels >> 2;  // 16-byte words per class row
+    const uint32_t words = (uint32_t) (p.bias_nrc * p.bias_ncc) * q4;
+    int4* dst = reinterpret_cast<int4*>(smem_raw + (smem_base - smem_u32(smem_raw)) + p.bias_off);
+    for (uint32_t i = (uint32_t) tid; i < words; i += kThreads) {
+      const uint32_t slot = i / q4, r = slot / (uint32_t) p.bias_ncc, c = slot - r * (uint32_t) p.bias_ncc;
+      const uint32_t cls = nibble(p.bias_rcls, r) * 8u + nibble(p.bias_ccls, c);
+      dst[i] = __ldg(reinterpret_cast<const int4*>(p.bias_cls) + cls * q4 + (i - slot * q4));
+    }
+  }
   tc_fence_before_sync();
   __syncthreads();
   tc_fence_after_sync();
@@ -497,7 +521,8 @@ __global__ void __launch_bounds__(kThreads, 1)
     // values that depend on the SPATIAL tile only: with the contiguous schedule (channel block fastest) they change once
     // every `cblocks` items, so they are recomputed only then
     bool row_ok = false;
-    uint32_t rm_row = 0;            // row class * 8 * channels: index of this lane's row of bias_cls, column class 0
+    uint32_t rm_row = 0;            // index of this lane's row of the bias table (row slot, column slot 0, channel 0)
+    const uint32_t bias_sbase = smem_base + (uint32_t) p.bias_off;
     for (uint32_t item = first; item < total; item += step) {
       const uint32_t empty_bar = smem_u32(&ctl.tmem_empty[as]);
       mbar_wait_parked(smem_u32(&ctl.tmem_full[as]), as_phase);
@@ -511,7 +536,7 @@ __global__ void __launch_bounds__(kThreads, 1)
         const int iy0 = oy * S - p.pad_top;
         const int rlo = iy0 < 0 ? -iy0 : 0, rhi = iy0 + 3 - p.in_h > 0 ? iy0 + 3 - p.in_h : 0;
         const uint32_t rm = rhi >= 3 ? 0u : (((7u << rlo) & 7u) & (7u >> rhi));
-        rm_row = rm * 8u * (uint32_t) p.channels;
+        rm_row = (SMB ? nibble(p.bias_rslot, rm) * (uint32_t) p.bias_rstride : rm * 8u) * (uint32_t) p.channels;
       }
       uint8_t* const obase = reinterpret_cast<uint8_t*>(it.tile_base) + it.c0;
       const uint32_t bias_row = rm_row + (uint32_t) it.c0;
@@ -532,14 +557,14 @@ __global__ void __launch_bounds__(kThreads, 1)
           // (item and sub-tile only); the general form costs ~25 instructions.
           const int ox_first = it.ox0 + 8 * j;
           if (ox_first * S - p.pad_left >= 0 && (ox_first + 7) * S - p.pad_left + 3 <= p.in_w) {
-            bias_idx = bias_row + 7u * (uint32_t) p.channels;
+            bias_idx = bias_row + (SMB ? nibble(p.bias_cslot, 7u) : 7u) * (uint32_t) p.channels;
             valid = row_ok;
           } else {
             const int ox = ox_first + px;
             const int ix0 = ox * S - p.pad_left;
             const int clo = ix0 < 0 ? -ix0 : 0, chi = ix0 + 3 - p.in_w > 0 ? ix0 + 3 - p.in_w : 0;
             const uint32_t cm = chi >= 3 ? 0u : (((7u << clo) & 7u) & (7u >> chi));
-            bias_idx = bias_row + cm * (uint32_t) p.channels;
+            bias_idx = bias_row + (SMB ? nibble(p.bias_cslot, cm) : cm) * (uint32_t) p.channels;
             valid = row_ok && ox < p.out_w;
           }
         }
@@ -564,10 +589,10 @@ __global__ void __launch_bounds__(kThreads, 1)
           // accumulator columns of (sub-tile j, group gi): pair mode keeps a pair's two groups side by side
           const uint32_t tlo = tbase + (PAIR ? (uint32_t) (gp * p.mt + j) * 32u : (uint32_t) (gi * p.mt + j) * NB);
           const uint32_t thi = PAIR ? tlo + 16u : tbase + (uint32_t) ((gi + 1) * p.mt + j) * NB;
-          const uint4 lo = epilogue_unit<RQ, NB>(p, tlo, p.bias_cls + (bias_idx + (uint32_t) gi * 16u), lastp && !two, empty_bar);
+          const uint4 lo = epilogue_unit<RQ, NB, SMB>(p, tlo, bias_idx + (uint32_t) gi * 16u, bias_sbase, lastp && !two, empty_bar);
           uint8_t* const dst = obase + (dst_off + (uint32_t) gi * 16u);
           if (two) {
-            const uint4 hi = epilogue_unit<RQ, NB>(p, thi, p.bias_cls + (bias_idx + (uint32_t) (gi + 1) * 16u), lastp, empty_bar);
+            const uint4 hi = epilogue_unit<RQ, NB, SMB>(p, thi, bias_idx + (uint32_t) (gi + 1) * 16u, bias_sbase, lastp, empty_bar);
             if (valid) {
               // (pixel strides that are odd multiples of 16 bytes — C = 144 — leave every other pixel 16-byte aligned only:
               // those lanes write their two halves separately, 1.5 instead of 2 requests per 32 bytes on average)
@@ -591,7 +616,7 @@ __global__ void __launch_bounds__(kThreads, 1)
           int j, gi;
           unit_split(un, it.mt_eff, inv, j, gi);
           sub_tile(j);
-          const uint4 o = epilogue_unit<RQ, NB>(p, tbase + (uint32_t) (gi * p.mt + j) * NB, p.bias_cls + (bias_idx + (uint32_t) gi * 16u),
+          const uint4 o = epilogue_unit<RQ, NB, SMB>(p, tbase + (uint32_t) (gi * p.mt + j) * NB, bias_idx + (uint32_t) gi * 16u, bias_sbase,
                                                 un + 4 >= units, empty_bar);
           if (valid) *reinterpret_cast<uint4*>(obase + (dst_off + (uint32_t) gi * 16u)) = o;
         }
@@ -618,14 +643,20 @@ static cudaError_t set_max_dynamic_smem(const void* kern, int max_smem_optin) {
   return cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, max_smem_optin - (int) fa.sharedSizeBytes);
 }
 
-template <int S, int RQ, int NB, bool PAIR = false>
-cudaError_t launch_one(const DwTcParams& p, const CUtensorMap& tm, int grid, int max_smem_optin, cudaStream_t stream) {
-  auto kern = q8_dwconv3x3_umma_kernel<S, RQ, NB, PAIR>;
+template <int S, int RQ, int NB, bool PAIR, bool SMB>
+cudaError_t launch_smb(const DwTcParams& p, const CUtensorMap& tm, int grid, int max_smem_optin, cudaStream_t stream) {
+  auto kern = q8_dwconv3x3_umma_kernel<S, RQ, NB, PAIR, SMB>;
   // once per instantiation, to the device maximum (a per-launch value raced between host threads; see the igemm launcher)
   static cudaError_t attr_status = set_max_dynamic_smem(reinterpret_cast<const void*>(kern), max_smem_optin);
   if (attr_status != cudaSuccess) return attr_status;
   kern<<<grid, kThreads, p.smem_total, stream>>>(p, tm);
   return cudaGetLastError();
+}
+
+template <int S, int RQ, int NB, bool PAIR = false>
+cudaError_t launch_one(const DwTcParams& p, const CUtensorMap& tm, int grid, int max_smem_optin, cudaStream_t stream) {
+  return p.bias_smem ? launch_smb<S, RQ, NB, PAIR, true>(p, tm, grid, max_smem_optin, stream)
+                     : launch_smb<S, RQ, NB, PAIR, false>(p, tm, grid, max_smem_optin, stream);
 }
 
 template <int S, int NB>

@@ -218,6 +218,40 @@ bool make_tmap_dw(CUtensorMap* tm, const uint8_t* in, size_t N, size_t H, size_t
 
 inline int idiv_floor(int a, int b) { return (a >= 0) ? a / b : -((-a + b - 1) / b); }
 
+// Border class bits of output position o along one axis (bit k: tap k lies inside [0, n)), as the depthwise epilogue computes them.
+inline uint32_t dw_border_bits(int o, int s, int pad, int n) {
+  const int i0 = o * s - pad;
+  const int lo = i0 < 0 ? -i0 : 0, hi = i0 + 3 - n > 0 ? i0 + 3 - n : 0;
+  return hi >= 3 ? 0u : (((7u << lo) & 7u) & (7u >> hi));
+}
+
+// Border-class biases of the depthwise tensor-core kernel (DwTcParams::bias_smem).  The epilogue reads 4 x 16 bytes of bias
+// per unit; from the global table (64 classes x C int32: 147 KB at C = 576, far more than the L1 left beside the kernel's
+// shared memory) those loads stall the requantisation — replacing them by a constant made 14x14x384 26 % and 7x7x960 23 %
+// faster (profiles/r3a_dw_layers.txt).  A geometry produces only the row classes of its output rows times the column classes
+// of its output columns (9 with padding <= 1 on images >= 3 pixels), so those rows of the table are copied into shared memory
+// wherever they fit beside the plan's ring and resident weights.  QNNP_CUDA_DW_BIAS_GLOBAL=1 keeps the global table.
+void plan_dw_bias_classes(q8::DwTcParams* p, int smem_limit) {
+  p->bias_smem = 0, p->bias_off = 0, p->bias_rstride = 8, p->bias_nrc = 8, p->bias_ncc = 8;
+  p->bias_rslot = p->bias_cslot = p->bias_rcls = p->bias_ccls = 0x76543210u;  // slot = class bits
+  uint32_t rset = 0, cset = 0;  // bit b set: class bits b occur
+  for (int oy = 0; oy < p->out_h; oy++) rset |= 1u << dw_border_bits(oy, p->stride, p->pad_top, p->in_h);
+  for (int ox = 0; ox < p->out_w; ox++) cset |= 1u << dw_border_bits(ox, p->stride, p->pad_left, p->in_w);
+  const int nrc = __builtin_popcount(rset), ncc = __builtin_popcount(cset);
+  const int bytes = nrc * ncc * p->channels * 4;
+  if (getenv("QNNP_CUDA_DW_BIAS_GLOBAL") != nullptr || p->smem_total + bytes > smem_limit) return;
+  uint32_t rslot = 0, cslot = 0, rcls = 0, ccls = 0;  // unproduced classes: slot 0
+  for (uint32_t b = 0, k = 0; b < 8; b++)
+    if (rset & (1u << b)) rslot |= k << (4 * b), rcls |= b << (4 * k), k++;
+  for (uint32_t b = 0, k = 0; b < 8; b++)
+    if (cset & (1u << b)) cslot |= k << (4 * b), ccls |= b << (4 * k), k++;
+  p->bias_smem = 1;
+  p->bias_off = p->smem_total - 1024;  // behind everything the plan placed (smem_total includes the 1024-byte alignment slack)
+  p->smem_total += bytes;
+  p->bias_rstride = ncc, p->bias_nrc = nrc, p->bias_ncc = ncc;
+  p->bias_rslot = rslot, p->bias_cslot = cslot, p->bias_rcls = rcls, p->bias_ccls = ccls;
+}
+
 // Tiling of the depthwise tensor-core kernel (q8_dwconv_umma_sm100.cu).  Pure function of the geometry, so that the
 // CPU test can replay the smem addressing it prescribes.  Returns false when the shape is not eligible.
 // pair != 0 plans the channel-pair form (see DwTcParams::pair); it needs a single weight operand (wmode != 2).
@@ -362,6 +396,7 @@ bool plan_dw_umma(int C, int batch, int H, int W, int OH, int OW, int s, int pad
   p->acc_stages = 2;
   p->total_items = (long long) p->nt * p->yt * p->xt * p->cblocks;
   if (p->total_items >= (1ll << 31)) return false;
+  plan_dw_bias_classes(p, smem_optin - kCtlReserve);
   return true;
 }
 
@@ -1277,6 +1312,16 @@ enum qnnp_status build_plan(qnnp_operator* op, const uint8_t* in, const uint8_t*
           (op->stride_h == 2 || env_set("QNNP_CUDA_DW_PAIR") || (tp.b_resident && tp.cgs >= 4)) &&
           make_tmap_dw(&pl.dw_tmap, in, op->batch, op->in_h, op->in_w, op->groups, op->in_stride, (int) op->stride_h, tp.box_px,
                        tp.box_rows, tp.nb, 1);
+      // ... except that at stride 1 the 16-channel form wins where only IT has room for the border-class table in shared
+      // memory (DwTcParams::bias_smem; 14x14x384: 0.257 ms in the pair form with the global table, 0.229 in the 16-channel
+      // form with the shared one)
+      if (tc_ok && op->stride_h == 1 && !tp.bias_smem && !env_set("QNNP_CUDA_DW_PAIR")) {
+        q8::DwTcParams t16;
+        if (plan_dw_umma((int) op->groups, (int) op->batch, (int) op->in_h, (int) op->in_w, (int) op->out_h, (int) op->out_w,
+                         (int) op->stride_h, (int) op->pad_top, (int) op->pad_left, op->dwtc_wmode, g_lib.max_smem_optin, &t16, 0) &&
+            t16.bias_smem)
+          tc_ok = false;
+      }
       if (!tc_ok)
         tc_ok = tc_base &&
             plan_dw_umma((int) op->groups, (int) op->batch, (int) op->in_h, (int) op->in_w, (int) op->out_h, (int) op->out_w,
@@ -1850,6 +1895,17 @@ QNNP_EXPORT int qnnp_cuda_debug_plan_dwconv32(int channels, int batch, int in_h,
                      1, p.a_off9[0], p.a_off9[1], p.a_off9[2], p.a_off9[3], p.a_off9[4], p.a_off9[5], p.a_off9[6], p.a_off9[7],
                      p.a_off9[8]};
   for (int i = 0; i < 48; i++) out[i] = v[i];
+  return 1;
+}
+/* Border-class bias table of the depthwise plan (either form), see qnnpack_cuda.h. */
+QNNP_EXPORT int qnnp_cuda_debug_plan_dwconv_bias(int channels, int batch, int in_h, int in_w, int out_h, int out_w, int stride,
+                                                 int pad_top, int pad_left, int wmode, int pair, int out[12]) {
+  q8::DwTcParams p;
+  const int optin = g_lib.initialized ? g_lib.max_smem_optin : 232448;
+  if (!plan_dw_umma(channels, batch, in_h, in_w, out_h, out_w, stride, pad_top, pad_left, wmode, optin, &p, pair)) return 0;
+  const int v[12] = {p.bias_smem, p.bias_off, p.bias_rstride, p.bias_nrc, p.bias_ncc, (int) p.bias_rslot, (int) p.bias_cslot,
+                     (int) p.bias_rcls, (int) p.bias_ccls, p.smem_total, p.num_stages, p.stage_bytes};
+  for (int i = 0; i < 12; i++) out[i] = v[i];
   return 1;
 }
 /* Channel-pair B operands (pack_dw_umma32_host): wpack must hold ceil(channels / 32) * 9 * 1024 bytes.  Returns the operand
